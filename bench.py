@@ -4,7 +4,7 @@ A "step" is ONE `model(batch)` call of the reference surface on synthetic pixels
 CLIP-ViT encoder -> visual projection -> image-row prefill of the 6 decoder layers -> KV-cached decode steps (max_len 40) ->
 search, i.e. the reference's `CaptioningModel.forward` in eval mode (reference layers/decoder.py:838-877, 977-1011).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2|3|4|5] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2|3|4|5] [--impl reference] [--dump-outputs DIR]
 
 --config names the BASELINE.json configuration (default 2 = the one the metric is quoted on):
   2  GIT_BASE,        64 images per call,            greedy   (BASELINE.json configs[1])
@@ -19,9 +19,15 @@ Numbers of a run (all with every call's full work inside the timed region):
   e2e     : the same calls with pinned HOST pixels in and token ids / logprobs read back to the host in every step.
   serving : (configs 2-4) the engine's asynchronous form `model.submit(batch, depth, coalesce)`: `coalesce` submitted batches
             share one engine launch, `depth` launches are in flight (dynamic batching: a serving technique, reported
-            beside the per-call metric, never in place of it).
+            beside the per-call metric, never in place of it).  It times K steps too: with K below depth * coalesce (8 for
+            configs 2 and 4 at the defaults) the pipeline never fills, so serving figures compare only at the same K.
 Multi-GPU (torchrun, one rank per GPU): every rank captions its own batches (weak scaling, image-wise sharding, reference
 inference.py:165-169); the timed region ends with ONE fused NCCL all_gather of all finished token ids + logprobs.
+`--dump-outputs DIR` writes what the last timed `value` step returned on rank 0 (its own shard, not the gathered
+captions) -- the token ids (float64, EOS-padded to 40 columns) and logprobs (float32) of its model(batch) calls -- as
+DIR/predictions.npy and DIR/logprobs.npy.  With `--impl reference` it writes the last timed CPU step instead: its
+`cpu_sample` images only, token ids not padded.  Weights and pixels are seeded, so two builds run with the same
+arguments can be compared output for output; the two arms' dumps are not the same images.
 `--impl reference` times the reference's own CPU algorithm (the as-shipped, no-KV-cache restatement in
 oracle/git_oracle.py -- the Python reference itself cannot travel to the GPU box) on the host cores.
 """
@@ -153,9 +159,18 @@ class ClockSampler(threading.Thread):
                 'samples': len(s)}
 
 
+def dump_outputs(dirname, predictions, logprobs):
+    """--dump-outputs: the arrays one timed step returned, token ids as float64 (exact) and logprobs as float32."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, 'predictions.npy'), predictions.cpu().numpy().astype(np.float64))
+    np.save(os.path.join(dirname, 'logprobs.npy'), logprobs.cpu().numpy().reshape(-1).astype(np.float32))
+
+
 def cpu_reference_runs(cfg, sample, steps, warmup):
     """The reference's CPU path as shipped (full [image || text] recompute every step), fp32: `warmup` untimed then `steps`
-    timed `model(batch)`-equivalents on `sample` images each.  Returns (captions/s, mean seconds per step, threads)."""
+    timed `model(batch)`-equivalents on `sample` images each.  Returns (captions/s, mean seconds per step, threads, the last
+    step's outputs)."""
     import torch
     sys.path.insert(0, os.path.join(ROOT, 'oracle'))
     import git_oracle
@@ -173,7 +188,7 @@ def cpu_reference_runs(cfg, sample, steps, warmup):
         if i >= warmup:
             times.append(dt)
     mean = sum(times) / len(times)
-    return sample / mean, mean, threads
+    return sample / mean, mean, threads, out
 
 
 def cpu_sample_text(cfg, sample, sec=None):
@@ -186,7 +201,9 @@ def run_reference_arm(args, cfg, rank):
     if rank != 0:
         return
     sample = cfg['cpu_sample']
-    value, sec, threads = cpu_reference_runs(cfg, sample, args.steps, args.warmup)
+    value, sec, threads, out = cpu_reference_runs(cfg, sample, args.steps, args.warmup)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out['predictions'], out['logprobs'])
     line = {
         'impl': 'reference', 'metric': cfg['metric'], 'value': value, 'unit': UNIT, 'n_gpus': args.gpus, 'steps': args.steps,
         'warmup': args.warmup, 'ms_per_step': sec * 1e3, 'higher_is_better': True, 'scaling': 'weak', 'vs_baseline': None,
@@ -220,6 +237,8 @@ def main():
                     help='serving leg: engine launches in flight (the encoder of launch i+1 overlaps the decode loop of launch i)')
     ap.add_argument('--coalesce', type=int, default=4, choices=[1, 2, 3, 4],
                     help='serving leg: this many submitted batches share one engine launch (at most 256 decoder rows)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the outputs of the last timed step as DIR/predictions.npy and DIR/logprobs.npy')
     ap.add_argument('--ncu-range', action='store_true',
                     help='bracket the timed region of `value` with cudaProfilerStart/Stop (use with ncu --profile-from-start off)')
     args = ap.parse_args()
@@ -307,6 +326,8 @@ def main():
                 keep(pend.pop(0).result())
         return toks, lps
 
+    last_step = {}
+
     def run(k, to_host=False, depth=1, coalesce=1, steps_per_call=1):
         """k steps; returns the per-step host-side completion times are not needed: events bracket the whole region."""
         src = host_batches if to_host else dev_batches
@@ -316,6 +337,7 @@ def main():
                 t, l = one_step(src, to_host, 1, 1)
                 all_t += t
                 all_l += l
+            last_step['outputs'] = (t, l)    # the tensors the step's calls returned (fresh per call: no copy needed)
         else:
             # serving leg: the k steps' batches are submitted back to back so that launches stay in flight across steps
             t, l = one_step(src * k, to_host, depth, coalesce)
@@ -365,6 +387,7 @@ def main():
         ms, launches = timed(args.steps)
         if args.ncu_range:
             torch.cuda.profiler.stop()
+        value_outputs = last_step['outputs']
         value = n_total * args.steps / (ms / 1e3)
         # ---------------- `e2e`: the same calls with HOST pixels in, tokens + logprobs back ----------------
         run(2, to_host=True)
@@ -378,7 +401,7 @@ def main():
         if not args.no_serving and args.config != 5:
             co = max(1, min(args.coalesce, 256 // (B * beam)))
             depth = args.pipeline
-            k_serv = max(args.steps, 2 * depth * co)
+            k_serv = args.steps
             run(2 * depth * co, depth=depth, coalesce=co)
             ms_s, _ = timed(k_serv, depth=depth, coalesce=co)
             run(2 * depth * co, to_host=True, depth=depth, coalesce=co)
@@ -461,9 +484,12 @@ def main():
     cpu = None
     if rank == 0 and not args.no_cpu_baseline:
         sample = {2: 12, 3: 3, 4: 2, 5: 6}[args.config]
-        v, sec, threads = cpu_reference_runs(cfg, sample, 1, 0)
+        v, sec, threads, _ = cpu_reference_runs(cfg, sample, 1, 0)
         cpu = {'value': v, 'unit': UNIT, 'cores': threads, 'host_cpus': os.cpu_count(), 'kind': 'port',
                'sample': 'one call, ' + cpu_sample_text(cfg, sample, sec)}
+
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, *(torch.cat(x, dim=0) for x in value_outputs))
 
     if rank == 0:
         steps_desc = ('one pass over the rank\'s %d-image shard in %d micro-batches of %d' % (shard, n_micro, B)) if n_micro > 1 \

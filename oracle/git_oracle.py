@@ -3,8 +3,9 @@ captioning hot path.  It is the *checker* for the CUDA engine and the `cpu_basel
 bench.py; the product package never imports it (the product fails loudly without its CUDA library).
 
 Parity status: the reference ships no tests or golden vectors (SURVEY.md section 4), so this
-restatement is pinned against the reference's own modules executed in the build container:
-  * tests/test_oracle_vs_reference.py runs both on the same seeded weights/pixels (needs /root/reference);
+restatement is pinned against outputs of the reference's own modules:
+  * tests/test_oracle_vs_reference.py compares it with what the reference returned on the same seeded weights/pixels
+    (tests/golden/reference_model.npz, recorded by oracle/make_reference_units.py);
   * tests/golden/*.npz were produced by the *unmodified reference* (oracle/make_golden.py) and are
     checked against this file on every machine (tests/test_oracle_golden.py).
 

@@ -1,9 +1,9 @@
 """TEST INFRASTRUCTURE ONLY -- imports the *unmodified* reference from /root/reference.
 
-Only usable in the build container (the GPU box has no /root/reference); it is used
-by oracle/make_golden.py to generate tests/golden/* and by
-tests/test_oracle_vs_reference.py to pin oracle/git_oracle.py against the reference's
-own modules.  Nothing in the product package may import this file.
+Only usable where the reference tree is present (REFERENCE_ROOT); it is used by
+oracle/make_golden.py and oracle/make_reference_units.py to record the reference's
+outputs as tests/golden/*, which the tests compare against.  Nothing in the product
+package may import this file.
 
 Shims (SURVEY.md section 8c / Appendix B):
   * `azfuse`, `boto3`, `botocore` are absent -> stub packages in oracle/stubs

@@ -1,4 +1,5 @@
 """Shared helpers for the parity tests (test infrastructure)."""
+import hashlib
 import json
 import os
 
@@ -6,6 +7,7 @@ import numpy as np
 import torch
 
 GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
+SAMPLE_STRIDE = 1021     # strided sample kept beside a digest where a full array would not fit a golden file
 
 
 def load_golden(name):
@@ -13,6 +15,17 @@ def load_golden(name):
     d = {k: g[k] for k in g.files}
     d['meta'] = json.loads(str(d['meta']))
     return d
+
+
+def digest(a):
+    """sha256 of an array's values in C order (with its dtype): bit-exact comparison against a stored reference output."""
+    a = a.detach().cpu().numpy() if isinstance(a, torch.Tensor) else np.asarray(a)
+    return hashlib.sha256(a.dtype.str.encode() + np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+def strided_sample(a):
+    a = a.detach().cpu().numpy() if isinstance(a, torch.Tensor) else np.asarray(a)
+    return np.ascontiguousarray(a).reshape(-1)[::SAMPLE_STRIDE].copy()
 
 
 def golden_inputs(meta):

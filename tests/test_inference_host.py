@@ -8,7 +8,7 @@ import pytest
 import torch
 
 import preprocess_oracle as po
-import ref_shim
+from helpers import load_golden
 from generativeimage2text_b200 import inference as inf
 from generativeimage2text_b200 import _lib
 
@@ -32,15 +32,16 @@ def test_geometry_equals_oracle_rules(param):
             assert (oh, ow) == (crop, crop)
 
 
-@pytest.mark.skipif(not ref_shim.reference_available(), reason='no /root/reference')
 def test_minmax_equals_reference_class():
-    ref_shim._import_reference()
-    import generativeimage2text.inference as rinf
-    for mn, mx in [(480, 640), (420, 560), (224, 224)]:
-        a, b = rinf.MinMaxResizeForTest(mn, mx), inf.MinMaxResizeForTest(mn, mx)
-        for h, w in SHAPES:
-            assert a.get_size((w, h)) == b.get_size((w, h))
-        assert repr(a) == repr(b)
+    """Sizes and repr against what the reference's MinMaxResizeForTest returned (stored by oracle/make_reference_units.py)."""
+    g = load_golden('reference_transform')['meta']['minmax']
+    assert [(c['min'], c['max']) for c in g] == [(480, 640), (420, 560), (224, 224)]
+    for c in g:
+        b = inf.MinMaxResizeForTest(c['min'], c['max'])
+        assert [s[:2] for s in c['sizes']] == [list(hw) for hw in SHAPES]
+        for h, w, want in c['sizes']:
+            assert list(b.get_size((w, h))) == want
+        assert repr(b) == c['repr']
 
 
 @pytest.mark.parametrize('pair', [(640, 298), (480, 224), (75, 224), (500, 720), (1920, 398), (3, 2), (5, 7), (224, 112),

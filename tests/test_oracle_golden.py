@@ -1,5 +1,5 @@
 """CPU: oracle/git_oracle.py against the golden vectors produced by the unmodified reference
-(oracle/make_golden.py).  This is what pins the oracle on machines without /root/reference."""
+(oracle/make_golden.py); with tests/test_oracle_vs_reference.py, this pins the oracle on every machine."""
 import numpy as np
 import pytest
 import torch

@@ -1,38 +1,43 @@
-"""CPU, build container only: oracle/git_oracle.py against the reference's own modules imported
-from /root/reference (skipped where the reference tree is absent, e.g. on the GPU box)."""
+"""CPU: oracle/git_oracle.py and the model's state-dict layout against what the reference's own modules returned on the
+same inputs (stored by oracle/make_reference_units.py)."""
 import pytest
 import torch
 
-import ref_shim
 import git_oracle
+from generativeimage2text_b200.model import get_git_model
 from generativeimage2text_b200.synthetic import state_spec, synthetic_state_dict, synthetic_images
+from helpers import load_golden
 
-pytestmark = pytest.mark.skipif(not ref_shim.reference_available(), reason='no /root/reference')
+
+class Tok:
+    cls_token_id, sep_token_id = 101, 102
 
 
 def test_state_dict_layout_matches_reference():
-    for param in ({}, {'num_image_with_embedding': 6}):
-        ref = ref_shim.load_reference_model(param, 'greedy', 40)
-        rsd = ref.state_dict()
+    for ref in load_golden('reference_model')['meta']['layout']:
+        param = ref['param']
         spec = state_spec(param)
-        assert [k for k, _, _ in spec] == list(rsd.keys())
-        for k, shp, _ in spec:
-            assert tuple(rsd[k].shape) == shp, k
-        assert rsd['textual.output.weight'].data_ptr() == rsd['textual.embedding.words.weight'].data_ptr()
+        assert [[k, list(shp)] for k, shp, _ in spec] == ref['keys']
+        # the same tensors share storage (the LM head is the word embedding)
+        groups = {}
+        for k, v in get_git_model(Tok(), param).state_dict().items():
+            groups.setdefault(v.data_ptr(), []).append(k)
+        assert [g for g in groups.values() if len(g) > 1] == ref['tied']
 
 
 @pytest.mark.parametrize('search', ['greedy', 'beam'])
 def test_oracle_equals_reference_fresh_seed(search):
-    """A seed/image set that is NOT in tests/golden: both implementations run here."""
-    sd = synthetic_state_dict({}, seed=7, variant='init')
-    img = synthetic_images(1, 0, seed=99)
-    ref = ref_shim.load_reference_model({}, search, 10, state_dict=sd)
-    with torch.no_grad():
-        r = ref({'image': img})
+    """A seed/image set that is NOT in tests/golden."""
+    g = load_golden('reference_model')
+    f = g['meta']['fresh']
+    sd = synthetic_state_dict({}, seed=f['weight_seed'], variant=f['variant'])
+    img = synthetic_images(1, 0, seed=f['img_seed'])
+    rp = torch.from_numpy(g['fresh_%s_predictions' % search])
+    rl = torch.from_numpy(g['fresh_%s_logprobs' % search])
     for cached in (True, False):
-        o = git_oracle.generate(sd, {}, {'image': img}, search, 10, cached=cached)
-        assert torch.equal(r['predictions'], o['predictions'])
-        assert torch.allclose(r['logprobs'], o['logprobs'], atol=1e-3)
+        o = git_oracle.generate(sd, {}, {'image': img}, search, f['max_steps'], cached=cached)
+        assert torch.equal(rp, o['predictions'])
+        assert torch.allclose(rl, o['logprobs'], atol=1e-3)
 
 
 # ---- the remaining decoders (SURVEY.md 8f-4): vocabulary trie, sampling ------------------------------------------------
@@ -51,26 +56,20 @@ def _toy_trie_sequences(eos):
     return [[5, 9, 11, eos], [5, 9, 12, 13, eos], [5, 20, eos], [7, 9, eos], [7, 30, 31, 32, eos], [40, eos]]
 
 
-def _import_trie_decoder():
-    ref_shim._import_reference()
-    import generativeimage2text.trie_decoder as td
-    return td
-
-
 def test_trie_search_equals_reference():
     """oracle/git_oracle.trie_search against the reference's TrieAutoRegressiveBeamSearch (trie_decoder.py:27-218) at batch 1,
     the case that decoder supports (with more rows its single cursor follows row 0 only and `TokenTrie.move` asserts as
     soon as row 0 has ended while another row has not): verbatim mode and the per-row mode the engine implements."""
     B = 1
     from generativeimage2text_b200.model import TokenTrie
-    td = _import_trie_decoder()
+    g = load_golden('reference_model')
     eos = 2
     seqs = _toy_trie_sequences(eos)
     start = torch.tensor([[1]] * B)
+    assert g['meta']['trie_seeds'] == 4
     for seed in range(4):
         step = _toy_step(seed=seed)
-        ref = td.TrieAutoRegressiveBeamSearch(eos, max_steps=12, beam_size=1, trie=td.TokenTrie.construct(seqs))
-        rp, rl = ref.search(start, step)
+        rp, rl = torch.from_numpy(g['trie_%d_predictions' % seed]), torch.from_numpy(g['trie_%d_logprobs' % seed])
         csr = TokenTrie.construct(seqs).to_csr()
         op, ol = git_oracle.trie_search(start, step, csr, max_steps=12, eos=eos, per_row=False)
         assert torch.equal(rp, op) and torch.allclose(rl, ol, atol=1e-5)
@@ -103,26 +102,15 @@ def test_trie_search_per_row_is_batch_of_batch1_calls():
 def test_sample_search_equals_reference_with_the_same_draws(temperature):
     """The do_sample branches of the reference's AutoRegressiveBeamSearch.search (layers/decoder.py:260-276, 364-375) with
     torch.multinomial replaced by the inverse-CDF draw the engine makes, fed the same uniforms."""
-    _, ref_decoder = ref_shim._import_reference()
+    g = load_golden('reference_model')
     eos, B, steps = 2, 4, 14
     start = torch.tensor([[1]] * B)
     u = torch.rand((steps, B), generator=torch.Generator().manual_seed(5))
+    assert g['meta']['sample_seeds'] == 3
     for seed in range(3):
         step = _toy_step(seed=seed)
-        dec = ref_decoder.AutoRegressiveBeamSearch(eos, max_steps=steps, beam_size=1, per_node_beam_size=1, fix_missing_prefix=True)
-        calls = {'t': start.shape[1]}
-
-        def fake_multinomial(probs, num_samples):
-            assert num_samples == 1
-            t = calls['t']
-            calls['t'] += 1
-            return git_oracle.inverse_cdf_draw(probs, u[t])[:, None]
-        real = torch.multinomial
-        torch.multinomial = fake_multinomial
-        try:
-            rp, rl = dec.search(start, step, do_sample=True, temperature=temperature)
-        finally:
-            torch.multinomial = real
+        rp = torch.from_numpy(g['sample_%g_%d_predictions' % (temperature, seed)])
+        rl = torch.from_numpy(g['sample_%g_%d_logprobs' % (temperature, seed)])
         op, ol = git_oracle.sample_search(start, step, u, temperature=temperature, max_steps=steps, eos=eos)
         assert torch.equal(rp, op)
         assert torch.allclose(rl, ol, atol=1e-5)

@@ -1,12 +1,12 @@
 """Pins oracle/preprocess_oracle.py (the CPU restatement of the reference's test-time transform, SURVEY.md section
 8f-2) against the third-party code the reference actually calls -- Pillow's resize and torchvision's transforms,
-executing here -- bit for bit; and against the reference's own `get_image_transform` / `MinMaxResizeForTest` when
-/root/reference is present."""
+executing here -- bit for bit; and against what the reference's own `get_image_transform` / `MinMaxResizeForTest`
+returned."""
 import numpy as np
 import pytest
 
 import preprocess_oracle as po
-import ref_shim
+from helpers import digest, load_golden, strided_sample
 
 PIL = pytest.importorskip('PIL')
 from PIL import Image  # noqa: E402
@@ -72,19 +72,18 @@ def test_full_transform_vs_torchvision_pipeline(param, hw):
     assert np.array_equal(got, want)
 
 
-@pytest.mark.skipif(not ref_shim.reference_available(), reason='no /root/reference')
 @pytest.mark.parametrize('param', [{}, {'test_crop_size': 480, 'test_respect_ratio_max': 640}])
 def test_equals_reference_get_image_transform(param):
-    ref_shim._import_reference()
-    import generativeimage2text.inference as rinf
-    t = rinf.get_image_transform(param)
-    for hw in [(480, 640), (1000, 300), (200, 200), (300, 1000), (480, 600)]:
-        img = _img(hw[0], hw[1], 3)
-        want = t(Image.fromarray(img)).numpy()
-        got = po.transform(img, param)
-        assert got.shape == want.shape
-        assert np.array_equal(got, want)
+    """Bit for bit against what the reference's own get_image_transform / MinMaxResizeForTest returned on these images
+    (stored by oracle/make_reference_units.py: shape, sha256 of the planes and a strided sample)."""
+    g = load_golden('reference_transform')
+    cases = [(k, c) for k, c in enumerate(g['meta']['transform']) if c['param'] == param]
+    assert len(cases) == 5
+    for k, c in cases:
+        got = po.transform(_img(c['hw'][0], c['hw'][1], c['img_seed']), param)
+        assert list(got.shape) == c['shape']
+        assert np.array_equal(strided_sample(got), g['transform_%d_sample' % k])
+        assert digest(got) == c['sha256']
         if 'test_respect_ratio_max' in param:
-            mm = rinf.MinMaxResizeForTest(param['test_crop_size'], param['test_respect_ratio_max'])
-            assert mm.get_size((hw[1], hw[0])) == po.minmax_size(hw[0], hw[1], param['test_crop_size'],
-                                                                   param['test_respect_ratio_max'])
+            assert list(po.minmax_size(c['hw'][0], c['hw'][1], param['test_crop_size'],
+                                       param['test_respect_ratio_max'])) == c['minmax_size']

@@ -1,14 +1,14 @@
 """Checkpoint ingestion (SURVEY.md section 8f-1): generativeimage2text_b200/torch_common.py against the reference's
-torch_common.py (run here when /root/reference is present) and against hand-checked cases everywhere."""
+torch_common.py (what it returned on the same inputs, stored under tests/golden) and against hand-checked cases."""
 import collections
 
 import pytest
 import torch
 
-import ref_shim
 from generativeimage2text_b200 import torch_common as tc
 from generativeimage2text_b200.model import get_git_model
 from generativeimage2text_b200.synthetic import synthetic_state_dict
+from helpers import digest, load_golden
 
 
 class Tok:
@@ -60,35 +60,34 @@ def test_load_state_dict_into_engine_shell(param):
     assert after['textual.output.weight'].data_ptr() == after['textual.embedding.words.weight'].data_ptr()
 
 
-@pytest.mark.skipif(not ref_shim.reference_available(), reason='no /root/reference')
 def test_same_result_as_reference_loader():
-    ref_shim._import_reference()
-    import generativeimage2text.torch_common as rtc
-    param = {'num_image_with_embedding': 6}
-    ckpt, _ = _messy_checkpoint(param)
-    ref = ref_shim.load_reference_model(param, 'stock')
+    """Every tensor ends up where the reference's torch_common.load_state_dict puts it: the checkpoint key it took, or the
+    model's own starting value (recorded by oracle/make_reference_units.py on the same checkpoint)."""
+    g = load_golden('reference_torch_common')['meta']['loader']
+    param = g['param']
+    ckpt, _ = _messy_checkpoint(param, g['ckpt_seed'])
     ours = get_git_model(Tok(), param)
     # same starting point for the tensors the checkpoint does not provide
-    start = synthetic_state_dict(param, 11, 'init')
-    ref.load_state_dict(start, strict=False)
+    start = synthetic_state_dict(param, g['start_seed'], 'init')
     ours.load_state_dict(start, strict=True)
-    rtc.load_state_dict(ref, ckpt)
     tc.load_state_dict(ours, ckpt)
-    rsd, osd = ref.state_dict(), ours.state_dict()
-    assert list(rsd.keys()) == list(osd.keys())
-    for k in rsd:
-        assert torch.equal(rsd[k], osd[k]), k
+    osd = ours.state_dict()
+    assert list(osd.keys()) == [k for k, _ in g['source']]
+    for k, src in g['source']:
+        assert torch.equal(osd[k], start[k] if src is None else ckpt[src]), k
 
 
-@pytest.mark.skipif(not ref_shim.reference_available(), reason='no /root/reference')
 @pytest.mark.parametrize('patch,width,after', [(16, 768, 480), (14, 1024, 420), (16, 768, 160)])
 def test_resize_2d_pos_embed_equals_reference(patch, width, after):
-    ref_shim._import_reference()
-    import generativeimage2text.torch_common as rtc
+    """Bit for bit against the reference's resize_2d_pos_embed output (sha256 stored by oracle/make_reference_units.py)."""
+    want = [c for c in load_golden('reference_torch_common')['meta']['pos_embed']
+            if (c['patch'], c['width'], c['after']) == (patch, width, after)]
+    assert len(want) == 1
+    want = want[0]
     g = 224 // patch
     pe = torch.randn(g * g + 1, width, generator=torch.Generator().manual_seed(5))
-    a = rtc.resize_2d_pos_embed(pe, 224, patch, after)
     b = tc.resize_2d_pos_embed(pe, 224, patch, after)
-    assert a.shape == b.shape == ((after // patch) ** 2 + 1, width)
-    assert torch.equal(a, b)
-    assert torch.equal(rtc.resize_2d_pos_embed(pe[None], 224, patch, after), tc.resize_2d_pos_embed(pe[None], 224, patch, after))
+    assert list(b.shape) == want['shape'] == [(after // patch) ** 2 + 1, width]
+    assert digest(b) == want['sha256']
+    b3 = tc.resize_2d_pos_embed(pe[None], 224, patch, after)
+    assert list(b3.shape) == want['shape_batched'] and digest(b3) == want['sha256_batched']

@@ -1,5 +1,5 @@
 """TSV container I/O (SURVEY.md section 8f-3): generativeimage2text_b200/tsv_io.py -- format checks everywhere, and
-byte-for-byte against the reference's tsv_io.py when /root/reference is present."""
+byte-for-byte against what the reference's tsv_io.py wrote for the same rows."""
 import base64
 import json
 import os
@@ -7,8 +7,8 @@ import os
 import numpy as np
 import pytest
 
-import ref_shim
 from generativeimage2text_b200 import tsv_io
+from helpers import load_golden
 
 
 def _rows(n, seed=0):
@@ -87,34 +87,30 @@ def test_concat_parts(tmp_path):
         assert t[i][0] == allrows[i][0] and t[i][1].encode() == allrows[i][1]
 
 
-@pytest.mark.skipif(not ref_shim.reference_available(), reason='no /root/reference')
 def test_byte_identical_to_reference_tsv_io(tmp_path):
-    ref_shim._import_reference()
-    import generativeimage2text.tsv_io as rio
-    rows = _rows(23, 7)
-    a, b = str(tmp_path / 'ours.tsv'), str(tmp_path / 'ref.tsv')
+    """Writer, reader and concat against what the reference's tsv_io.py produced for the same rows (stored by
+    oracle/make_reference_units.py)."""
+    g = load_golden('reference_tsv_io')
+    rows = _rows(*g['meta']['rows'])
+    a = str(tmp_path / 'ours.tsv')
     tsv_io.tsv_writer(iter(rows), a)
-    rio.tsv_writer(iter(rows), b)
-    for fa, fb in zip(_files(a), _files(b)):
-        assert open(fa, 'rb').read() == open(fb, 'rb').read(), fa
-    ours_on_ref, ref_on_ours = tsv_io.TSVFile(b), rio.TSVFile(a)
-    assert len(ours_on_ref) == len(ref_on_ours) == 23
-    for i in (0, 22, 9):
-        assert ours_on_ref[i] == ref_on_ours[i]
-        assert ours_on_ref.get_key(i) == ref_on_ours.get_key(i)
-    # merged parts: same .tsv and .lineidx.8b as the reference's concat (its process pool is bypassed: num_worker=0)
+    for fa, ext in zip(_files(a), ('tsv', 'lineidx', 'lineidx_8b')):
+        assert open(fa, 'rb').read() == g['written_' + ext].tobytes(), fa
+    b = str(tmp_path / 'ref.tsv')
+    for fb, ext in zip(_files(b), ('tsv', 'lineidx', 'lineidx_8b')):
+        with open(fb, 'wb') as fp:
+            fp.write(g['written_' + ext].tobytes())
+    ours_on_ref = tsv_io.TSVFile(b)
+    assert len(ours_on_ref) == len(rows)
+    for i, ref_read in g['meta']['reads'].items():
+        assert ours_on_ref[int(i)] == ref_read['row']
+        assert ours_on_ref.get_key(int(i)) == ref_read['key']
+    # merged parts: same .tsv and .lineidx.8b as the reference's concat
+    split = g['meta']['split']
     p1, p2 = str(tmp_path / 'p.0.2.tsv'), str(tmp_path / 'p.1.2.tsv')
-    tsv_io.tsv_writer(iter(rows[:10]), p1)
-    tsv_io.tsv_writer(iter(rows[10:]), p2)
-    o1, o2 = str(tmp_path / 'm_ours.tsv'), str(tmp_path / 'm_ref.tsv')
+    tsv_io.tsv_writer(iter(rows[:split]), p1)
+    tsv_io.tsv_writer(iter(rows[split:]), p2)
+    o1 = str(tmp_path / 'm_ours.tsv')
     tsv_io.concat_tsv_files([p1, p2], o1)
-    orig = rio.parallel_map
-    rio.parallel_map = lambda f, tasks, num_worker=0: [f(t) for t in tasks]
-    os.environ['GIT_TMP_FOLDER'] = str(tmp_path / 'tmp')
-    os.makedirs(os.path.join(os.environ['GIT_TMP_FOLDER'], str(tmp_path).lstrip('/')), exist_ok=True)
-    try:
-        rio.concat_tsv_files([p1, p2], o2)
-    finally:
-        rio.parallel_map = orig
-    assert open(o1, 'rb').read() == open(o2, 'rb').read()
-    assert open(_files(o1)[2], 'rb').read() == open(_files(o2)[2], 'rb').read()
+    assert open(o1, 'rb').read() == g['merged_tsv'].tobytes()
+    assert open(_files(o1)[2], 'rb').read() == g['merged_lineidx_8b'].tobytes()
